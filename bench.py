@@ -3,6 +3,7 @@
     python bench.py --gpus 1 --steps 10 --warmup 3                    # this build (CUDA, sm_100a)
     python bench.py --impl reference --gpus 1 --steps 3 --warmup 1    # the reference's CPU arithmetic (oracle port)
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
+    python bench.py --gpus 1 --steps 10 --warmup 3 --dump-outputs DIR  # + what the last timed step computed, as .npy
 
 Workload at N=1: BASELINE.json configs[1] ("cfg2"): VisualBERT-base 12L/768H, COCO masked-LM pretrain step
 (MLM + NSP heads), batch 256, 36 regions (2048-d) + 128 tokens, bf16, train mode (dropout active).
@@ -29,6 +30,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 from visualbert_b200 import synthetic  # noqa: E402
@@ -163,7 +165,7 @@ def run_reference(args):
         return 0
     c = build_cfg(args.config)
     sample_b = args.cpu_sample
-    dt, threads, spread = cpu_oracle_step_time(c, sample_b, max(args.steps, 5), args.warmup, threads=cpu_threads())
+    dt, threads, spread = cpu_oracle_step_time(c, sample_b, args.steps, args.warmup, threads=cpu_threads())
     value = sample_b / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -178,6 +180,31 @@ def run_reference(args):
     }
     print(json.dumps(line))
     return 0
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, outputs, model):
+    """Write what one step handed back as float32 .npy files under `out_dir`: every output tensor of the forward pass
+    (`<key>.npy`, in full) and every parameter's gradient (`grad.<parameter name>.npy`), the latter at positions drawn
+    from a fixed seed wherever a gradient is too large to fit its share of the 64 MB the whole dump may take."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in outputs.items()}
+    named = [(n, p.grad.detach().reshape(-1)) for n, p in model.named_parameters() if p.grad is not None]
+    header = 4096   # per file: the .npy header, with room to spare
+    per_grad = ((DUMP_BYTES - sum(a.nbytes + header for a in arrays.values())) // len(named) - header) // 4
+    gen = torch.Generator().manual_seed(0)
+    for name, g in named:
+        if g.numel() > per_grad:
+            idx = torch.randint(g.numel(), (per_grad,), generator=gen).sort().values
+            g = g[idx.to(g.device)]
+        arrays["grad." + name] = g.float().cpu().numpy()
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    total = sum(os.path.getsize(os.path.join(out_dir, k + ".npy")) for k in arrays)
+    assert total <= DUMP_BYTES, total
+    return len(arrays), total
 
 
 def workload_name(c):
@@ -226,12 +253,17 @@ def run_ours(args):
     h2d_bytes = sum(v.numel() * v.element_size() for v in resident.values() if torch.is_tensor(v))
 
     lscale = sync.loss_scale()   # 1 / world: the mean over ranks is folded into the loss, no divide pass over the buffer
+    last = {}   # --dump-outputs: the output tensors of the latest step
 
     def step(batch):
         sync.zero()
         out = model(**batch)
         (out["loss"] * lscale if world > 1 else out["loss"]).backward()
         sync.allreduce(prescaled=True)
+        if args.dump_outputs:
+            # dict.items: the entries as stored; a lazy one the step never read (the MLM logits) is None, not computed
+            last.clear()
+            last.update((k, v) for k, v in dict.items(out) if torch.is_tensor(v))
         if opt is not None:
             opt.step()
         return out["loss"]
@@ -265,6 +297,8 @@ def run_ours(args):
         clk.mark()
         ms_total = timed(lambda: step(resident), args.steps)
         launches = _lib.launch_count() - n0
+        if args.dump_outputs and rank == 0:   # before the passes below overwrite the gradients
+            dumped = dump_outputs(args.dump_outputs, last, model)
         # ---- roofline pass: the SAME K steps again with a CUDA-event pair around every launch of the library ----
         _lib.profile_read()
         _lib.profile_enable(True)
@@ -421,6 +455,9 @@ def run_ours(args):
         "e2e": {"value": e2e_value, "unit": UNIT, "ms_per_step": ms_e2e, "h2d_bytes_per_step": int(h2d_bytes),
                 "d2h_bytes_per_step": 4, "host_enqueue_ms_per_step": round(1e3 * enq[0] / max(1, enq[1]), 3)},
     }
+    if args.dump_outputs:
+        line["dump_outputs"] = {"dir": args.dump_outputs, "files": dumped[0], "bytes": dumped[1],
+                                "of": f"the last of the {args.steps} timed steps"}
     if opt_info is not None:
         line["optimizer"] = opt_info
     if others is not None:
@@ -450,7 +487,14 @@ def main():
                     help="also time BASELINE.json configs[2..4] at their per-GPU batch (always on for N > 1)")
     ap.add_argument("--optimizer", action="store_true",
                     help="also run the fused BertAdam step every step (SURVEY §8f rank 2; the BASELINE metric excludes it)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (outputs, sampled gradients) as "
+                         "DIR/<name>.npy, float32, 64 MB at most")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

@@ -81,6 +81,8 @@ def main():
     M = import_reference()
     out_dir = os.path.join(ROOT, "tests", "golden")
     os.makedirs(out_dir, exist_ok=True)
+    if "--only-wrapper" in sys.argv:
+        return make_wrapper_golden(out_dir)
     make_bert_adam_golden(out_dir)
     if "--only-adam" in sys.argv:
         return
@@ -148,6 +150,161 @@ def main():
             rec["grad_sub::" + k] = subsample(dict(model.named_parameters())[k].grad)
         np.savez_compressed(os.path.join(out_dir, name + ".npz"), **rec)
         print(f"{name}: loss={loss.item():.6f} logits{tuple(logits.shape)} -> {name}.npz")
+    if not only:
+        make_wrapper_golden(out_dir)
+
+
+WRAPPER_CASES = ("small_nlvr", "small_vqa", "small_ragged_pretraining")
+MODEL_DIR = "<bert_model_dir>"   # stands for the model directory the wrapper was handed
+
+
+def _install_wrapper_standins(objective_cls):
+    """allennlp.* names model.py:11-18 imports (AllenNLP 0.8 is not installable offline, SURVEY.md §8c); only Model (an
+    nn.Module with a `register` decorator and a vocab) and the two metrics the wrapper instantiates need behaviour.
+    pytorch_pretrained_bert.modeling serves `objective_cls`: the one-line import swap of INTEGRATION.md §1 (model.py:20).
+    Returns the sys.modules entries it replaced."""
+
+    class Model(torch.nn.Module):
+        def __init__(self, vocab=None):
+            super().__init__()
+            self.vocab = vocab
+
+        @classmethod
+        def register(cls, name):
+            return lambda klass: klass
+
+    class CategoricalAccuracy:
+        def __init__(self):
+            self.correct, self.total = 0.0, 0.0
+
+        def __call__(self, logits, labels):
+            self.correct += (logits.argmax(-1).view(-1) == labels.view(-1)).float().sum().item()
+            self.total += labels.numel()
+
+        def get_metric(self, reset=False):
+            v = self.correct / max(self.total, 1.0)
+            if reset:
+                self.correct = self.total = 0.0
+            return v
+
+    class Average:
+        def __init__(self):
+            self.s, self.n = 0.0, 0
+
+        def __call__(self, v):
+            self.s += float(v); self.n += 1
+
+        def get_metric(self, reset=False):
+            v = self.s / max(self.n, 1)
+            if reset:
+                self.s, self.n = 0.0, 0
+            return v
+
+    anything = type("Anything", (), {})
+    mods = {
+        "allennlp": {}, "allennlp.data": {}, "allennlp.data.vocabulary": dict(Vocabulary=anything),
+        "allennlp.models": {}, "allennlp.models.model": dict(Model=Model),
+        "allennlp.modules": dict(TextFieldEmbedder=anything, Seq2SeqEncoder=anything, FeedForward=anything,
+                                 InputVariationalDropout=anything, TimeDistributed=anything),
+        "allennlp.training": {}, "allennlp.training.metrics": dict(CategoricalAccuracy=CategoricalAccuracy, Average=Average),
+        "allennlp.modules.matrix_attention": dict(BilinearMatrixAttention=anything),
+        "allennlp.nn": dict(InitializerApplicator=anything),
+        "allennlp.nn.util": dict(masked_softmax=None, weighted_sum=None, replace_masked_values=None),
+        "pytorch_pretrained_bert": {},
+        "pytorch_pretrained_bert.modeling": dict(TrainVisualBERTObjective=objective_cls, BertForMultipleChoice=anything),
+        "pytorch_pretrained_bert.file_utils": dict(PYTORCH_PRETRAINED_BERT_CACHE="pretrained_cache"),
+    }
+    saved = {name: sys.modules.get(name) for name in mods}
+    for name, attrs in mods.items():
+        m = types.ModuleType(name)
+        for k, v in attrs.items():
+            setattr(m, k, v)
+        sys.modules[name] = m
+    return saved
+
+
+def make_wrapper_golden(out_dir):
+    """The reference's AllenNLP wrapper `visualbert/models/model.py:191-306` (VisualBERTFixedImageEmbedding), executed
+    unmodified on visualbert_b200.TrainVisualBERTObjective, with the oracle's (sequence_output, pooled_output) standing
+    in for the CUDA encoder. Records every call the wrapper makes into the objective (from_pretrained arguments,
+    special_intialize, the forward keywords with their tensors) and what the wrapper returns (output keys, loss,
+    accuracy metric): tests/test_wrapper_dropin_cpu.py replays the calls and checks the results."""
+    import json
+    import tempfile
+
+    import vb_oracle
+    import visualbert_b200
+    from visualbert_b200 import BertConfig
+    from visualbert_b200.modeling import BertEmbeddingsWithVisualEmbedding
+
+    calls = []
+
+    class RecordingObjective(visualbert_b200.TrainVisualBERTObjective):
+        @classmethod
+        def from_pretrained(cls, *args, **kwargs):
+            calls.append(dict(name="from_pretrained", args=args, kwargs=kwargs))
+            return super().from_pretrained(*args, **kwargs)
+
+        def forward(self, **kwargs):
+            calls.append(dict(name="forward", kwargs=kwargs))
+            return super().forward(**kwargs)
+
+    special_init = BertEmbeddingsWithVisualEmbedding.special_intialize
+
+    def recording_special_init(self, *args, **kwargs):
+        calls.append(dict(name="special_intialize", args=args, kwargs=kwargs))
+        return special_init(self, *args, **kwargs)
+
+    saved = _install_wrapper_standins(RecordingObjective)
+    BertEmbeddingsWithVisualEmbedding.special_intialize = recording_special_init
+    try:
+        path = os.path.join(REF, "models", "model.py")
+        ns = {"__name__": "reference_models_model"}
+        exec(compile(open(path).read(), path, "exec"), ns)
+        for name in WRAPPER_CASES:
+            cfg, sd, batch, c = build_case(name)
+            calls.clear()
+            with tempfile.TemporaryDirectory() as model_dir:
+                with open(os.path.join(model_dir, "bert_config.json"), "w") as f:
+                    f.write(BertConfig.from_dict(cfg).to_json_string())
+                m = ns["VisualBERTFixedImageEmbedding"](vocab=None, bert_model_name=model_dir, training_head_type=c["head"],
+                                                        visual_embedding_dim=c["Dv"], random_initialize=True,
+                                                        special_visual_initialize=True)
+                calls[0]["args"] = [MODEL_DIR if a == model_dir else a for a in calls[0]["args"]]
+            res = m.bert.load_state_dict(sd, strict=False)
+            assert set(res.missing_keys) <= {"cls.predictions.decoder.weight"} and not res.unexpected_keys, res
+            m.eval()
+            kw = {k: v for k, v in batch.items() if k != "position_embeddings_visual"}
+            with torch.no_grad():
+                ref = vb_oracle.objective(sd, cfg, c["head"], **kw)
+            m.bert.bert.forward = lambda *a, **k: (ref["sequence_output"], ref["pooled_output"])
+            image_dim = batch["image_mask"].sum(-1)   # the wrapper rebuilds image_mask from the region count (model.py:262-268)
+            out = m(bert_input_ids=batch["input_ids"], bert_input_mask=batch["input_mask"],
+                    bert_input_type_ids=batch["token_type_ids"], image_dim_variable=image_dim,
+                    image_feat_variable=batch["visual_embeddings"], visual_embeddings_type=batch.get("visual_embeddings_type"),
+                    label=batch.get("label"), masked_lm_labels=batch.get("masked_lm_labels"),
+                    is_random_next=batch.get("is_random_next"))
+            assert [x["name"] for x in calls] == ["from_pretrained", "special_intialize", "forward"], calls
+            rec = {}
+            fwd = calls[2]["kwargs"]
+            for k, v in fwd.items():
+                if torch.is_tensor(v):
+                    rec["forward::" + k] = v.detach().numpy()
+            meta = dict(
+                from_pretrained=dict(args=calls[0]["args"], kwargs=calls[0]["kwargs"]),
+                special_intialize=dict(args=calls[1]["args"], kwargs=calls[1]["kwargs"]),
+                forward_values={k: v for k, v in fwd.items() if not torch.is_tensor(v)},
+                output_keys=sorted(out.keys()), loss=out["loss"].item(), accuracy=m.get_metrics(reset=True)["accuracy"])
+            rec["calls"] = np.array(json.dumps(meta, sort_keys=True))
+            np.savez_compressed(os.path.join(out_dir, f"wrapper_{name}.npz"), **rec)
+            print(f"wrapper_{name}: loss={meta['loss']:.6f} accuracy={meta['accuracy']:.4f} -> wrapper_{name}.npz")
+    finally:
+        BertEmbeddingsWithVisualEmbedding.special_intialize = special_init
+        for name, mod in saved.items():
+            if mod is None:
+                sys.modules.pop(name, None)
+            else:
+                sys.modules[name] = mod
 
 
 def make_bert_adam_golden(out_dir):

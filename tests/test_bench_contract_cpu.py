@@ -6,6 +6,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import torch
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -21,7 +24,30 @@ def test_reference_arm_prints_one_json_line_with_the_contract_keys():
               "cpu_baseline", "e2e"):
         assert k in d, k
     assert d["value"] > 0 and d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["value"] == d["value"]
+    assert d["steps"] == 1 and d["cpu_baseline"]["spread"]["steps"] == 1   # --steps is the number of timed steps
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0 and d["e2e"]["value"] == d["value"]
+
+
+def test_dump_outputs_writes_float32_seeded_samples_within_64_mb(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    torch.manual_seed(0)
+    model = torch.nn.Sequential(torch.nn.Embedding(30522, 768), torch.nn.Linear(768, 768))  # 94 MB of fp32 gradient
+    for p in model.parameters():
+        p.grad = torch.randn_like(p)
+    outputs = {"loss": torch.tensor(1.5), "seq_relationship_score": torch.randn(4, 2).bfloat16()}
+    n, total = bench.dump_outputs(str(tmp_path / "a"), outputs, model)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert n == len(files) == 5 and total <= 64 << 20
+    assert files == ["grad.0.weight.npy", "grad.1.bias.npy", "grad.1.weight.npy", "loss.npy", "seq_relationship_score.npy"]
+    a = {f: np.load(tmp_path / "a" / f) for f in files}
+    assert all(x.dtype == np.float32 for x in a.values())
+    assert a["loss.npy"] == 1.5 and np.array_equal(a["seq_relationship_score.npy"], outputs["seq_relationship_score"].float().numpy())
+    assert np.array_equal(a["grad.1.weight.npy"], model[1].weight.grad.reshape(-1).numpy())   # small enough: whole
+    big = a["grad.0.weight.npy"]
+    assert 0 < big.size < model[0].weight.numel() and np.isin(big, model[0].weight.grad.numpy()).all()
+    bench.dump_outputs(str(tmp_path / "b"), outputs, model)
+    assert all(np.array_equal(np.load(tmp_path / "b" / f), a[f]) for f in files)   # the same positions every time
 
 
 def test_per_gpu_batch_of_the_eight_gpu_configs():
