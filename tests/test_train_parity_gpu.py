@@ -44,11 +44,19 @@ def hidden_keep(seed, stream, rows, cols, p, dev):
     return (byte >= n).view(rows, cols), 256.0 / (256.0 - n)
 
 
-@pytest.mark.parametrize("B,S,A,layer_index", [(3, 164, 4, 0), (2, 100, 2, 5), (2, 56, 2, 11)])
+# The last four rows are BERT-base width (H = 768, A = 12) at B = 64, i.e. 768 attention items: >= 5 per CTA of the persistent
+# attention kernels on a 148-SM B200. S = 164 is the benchmark geometry (B*S a multiple of 256: tile-native gelu', fused
+# rowsum(dO * O) in the dO GEMM epilogue); S = 185 takes the 1-stage tcgen05 backward, the fused rowsum with an odd sequence
+# length and the row-major gelu'; S = 76 a single query tile; S = 200 the whole-head kernels.
+@pytest.mark.parametrize("B,S,A,layer_index", [(3, 164, 4, 0), (2, 100, 2, 5), (2, 56, 2, 11),
+                                               (64, 164, 12, 3), (64, 185, 12, 7), (64, 76, 12, 1), (64, 200, 12, 9)])
 def test_layer_train_mode_matches_reference_math_with_the_same_masks(B, S, A, layer_index):
     from visualbert_b200 import _lib
     L = _lib.lib()
     dev = torch.device("cuda:0")
+    if B * A >= 256:   # the production-scale rows: many attention items per CTA, and uneven counts
+        sms = torch.cuda.get_device_properties(0).multi_processor_count
+        assert B * A >= 5 * sms and B * A % sms != 0, (B * A, sms)
     st = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
     torch.manual_seed(17 + layer_index)
     H, I = A * 64, A * 256

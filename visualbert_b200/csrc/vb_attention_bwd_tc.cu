@@ -249,6 +249,12 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
                     while (next_sd < n_units && next_sd <= g + 2) {
                         const int li = next_sd / upi, ul = next_sd - li * upi, kt = ul / nqb, qb = ul - kt * nqb;
                         if (nstage == 1 && li > (g < 0 ? 0 : li_g + (item_end ? 1 : 0))) break;   // its inputs are not released yet
+                        // its element-wise pass overwrites dS^T atom qb of tile kt, which the previous item's dQ MMA reads at
+                        // unit (qb | 1) or nqb - 1 of that tile: issue after that MMA, so SD_FULL (in-order completion) also
+                        // means the atom is free.
+                        // Binds only with one or two units per item (S <= 128); it also keeps the shared ACC_FULL / DQ_FULL
+                        // waits of the two warp-groups in phase order when every item has a single unit.
+                        if (next_sd - upi + min(qb | 1, nqb - 1) - qb > g) break;
                         const int s = li % nstage, slot = next_sd & 1;
                         const int bw = min(64, npq - 64 * qb);
                         if (ul == 0) {
